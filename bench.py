@@ -29,6 +29,7 @@ per patch, numpy blend with the reference's whole-volume copies; validated at 0.
 tests/golden/time_reference_cpu.py) on ALL host cores (torch's thread count is set explicitly: torchrun exports
 OMP_NUM_THREADS=1), on a bounded sample of patches of the same workload; its line carries the CPU training step as `train`.
 `--task train` prints the training record as a line of its own.
+`--dump-outputs DIR` writes what the last timed step returned (see write_outputs) for comparing two builds output for output.
 """
 import argparse
 import json
@@ -37,6 +38,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True       # the benchmark may run from a read-only tree and writes nothing into it
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, 'medical-segmentation3d-toolkit_b200')
@@ -155,6 +158,37 @@ class ClockSampler(object):
         sm.sort()
         med = sm[len(sm) // 2] if sm else None
         return {'sm_mhz': med, 'sm_max_mhz': smax, 'reasons': sorted(reasons), 'samples': len(sm)}
+
+
+DUMP_INFER_BYTES = 48 << 20   # sampled probabilities + mask of the last inference step
+DUMP_PARAMS = 1 << 20         # sampled parameter values after the last training step (4 MB): the dump stays under 64 MB
+
+
+def flat_sample(n, k, device):
+    """Flat indices into an output of n elements: all of them when n <= k, otherwise about k sorted distinct ones drawn
+    from a fixed seed, so every run and every build samples the same elements."""
+    if n <= k:
+        return torch.arange(n, device=device)
+    return torch.from_numpy(np.unique(np.random.default_rng(0).integers(0, n, k))).to(device)
+
+
+def sample_infer_outputs(probs, mask):
+    """(probabilities [C, ...] fp32, label mask int8) of one sliding-window pass -> float32 host arrays [C, k] and [k]."""
+    C = probs.shape[0]
+    k = DUMP_INFER_BYTES // (4 * (C + 1))
+    p, m = probs.reshape(C, -1), mask.reshape(-1)
+    return {'infer_probs': p[:, flat_sample(p.shape[1], k, p.device)].float().cpu().numpy(),
+            'infer_mask': m[flat_sample(m.numel(), k, m.device)].float().cpu().numpy()}
+
+
+def write_outputs(path, arrays):
+    """DIR/<name>.npy per array: infer_probs / infer_mask (a fixed sample of the voxels of the last timed inference
+    step), train_loss and train_params (the loss and a fixed sample of the flattened parameters after the last timed
+    training step)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def peaks():
@@ -317,11 +351,17 @@ def measure_train(args, dist, rank, world, dev, cpu_leg=True):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     loss_value = float(loss.item())
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        flat = torch.cat([p.detach().reshape(-1).float() for p in params])
+        outputs = {'train_loss': np.array([loss_value], np.float64),
+                   'train_params': flat[flat_sample(flat.numel(), DUMP_PARAMS, flat.device)].cpu().numpy()}
+        del flat
     resolved = net.resolve_mode(train=True)
     del net, opt, crops, masks
     torch.cuda.empty_cache()
     if rank != 0:
-        return None
+        return None, None
     _, _, tf_sust, which = peaks()
     flops = 3.0 * VNET_GFLOP_PER_PATCH * 1e9 * B * (P / 96.0) ** 3        # forward + data gradient + weight gradient, per GPU
     rec = {
@@ -338,7 +378,7 @@ def measure_train(args, dist, rank, world, dev, cpu_leg=True):
     }
     if cpu_leg and world == 1 and not args.no_cpu_baseline:
         rec['cpu_baseline'] = cpu_train_record(args)
-    return rec
+    return rec, outputs
 
 
 def run_train(args):
@@ -350,9 +390,11 @@ def run_train(args):
     dist = None
     if world > 1:
         dist = init_nccl(dev)
-    rec = measure_train(args, dist, rank, world, dev)
+    rec, outputs = measure_train(args, dist, rank, world, dev)
     if rank == 0:
         rec['vs_baseline'] = None
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(rec))
     if dist is not None:
         dist.destroy_process_group()
@@ -390,7 +432,14 @@ def main():
     ap.add_argument('--train-batch', type=int, default=8)
     ap.add_argument('--arch', default='vnet', choices=['vnet', 'vbnet'], help='vbnet + --classes 5 = BASELINE configs[3]')
     ap.add_argument('--classes', type=int, default=2)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned to DIR/<name>.npy (float32/float64, under 64 MB: fixed seeded '
+                         'samples of the larger outputs; the inputs are the same in every run)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs records the GPU path; --impl reference has no such outputs')
     world = int(os.environ.get('WORLD_SIZE', '1'))
     if args.shard is None:
         args.shard = 'patches' if max(world, args.gpus if args.impl == 'reference' else 1) > 1 else 'cases'
@@ -439,7 +488,8 @@ def main():
         l0 = model['engine'].kernel_launches
         e0.record()
         for _ in range(steps):
-            fn()
+            out = None          # the previous step's outputs go back to the allocator before the next step allocates its own
+            out = fn()
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -448,29 +498,31 @@ def main():
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms / steps, launches
+        return ms / steps, launches, out
 
     def measure(shard_mode):
         shard = (rank, world) if (shard_mode == 'patches' and world > 1) else None
-        ms_dev, launches = timed(lambda: segmentation_volume_device(model, cfg, vol, batch=args.batch, shard=shard, gather=args.gather),
-                                 args.steps, max(args.warmup, 3))
+        ms_dev, launches, out = timed(lambda: segmentation_volume_device(model, cfg, vol, batch=args.batch, shard=shard, gather=args.gather),
+                                      args.steps, max(args.warmup, 3))
         # sharded: the merged mask is reduced to rank 0, the one process that copies it out (and would write the result file)
-        ms_e2e, _ = timed(lambda: segmentation_volume_host(model, cfg, host_vol, host_mask, batch=args.batch, shard=shard, gather=args.gather,
-                                                           mask_root=0 if shard is not None else None),
-                          max(2, args.steps // 2), 3)
+        ms_e2e, _, _ = timed(lambda: segmentation_volume_host(model, cfg, host_vol, host_mask, batch=args.batch, shard=shard, gather=args.gather,
+                                                              mask_root=0 if shard is not None else None),
+                             args.steps, 3)
         units = nvox * (world if shard is None else 1)
         return {'value': units / (ms_dev * 1e-3) / 1e6, 'ms_per_step': ms_dev, 'launches': launches,
-                'e2e': units / (ms_e2e * 1e-3) / 1e6, 'ms_e2e': ms_e2e}
+                'e2e': units / (ms_e2e * 1e-3) / 1e6, 'ms_e2e': ms_e2e}, out
 
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    head = measure(args.shard)
+    head, last = measure(args.shard)
     clocks = sampler.stop() if rank == 0 else None
+    dump = sample_infer_outputs(*last) if (args.dump_outputs and rank == 0) else {}
+    del last
     weak = None
     if world > 1 and args.shard == 'patches' and not args.no_weak:
         # every rank its own copy of the volume: replicas only, no collective on the data path
-        weak = measure('cases')
+        weak, _ = measure('cases')
 
     # parity of this very run: the device result of the single-GPU pass against the CPU reference on the sampled patches
     parity, cpu = None, None
@@ -558,7 +610,9 @@ def main():
         net._plans.clear()
         net._plan = None
         torch.cuda.empty_cache()
-        train = measure_train(args, dist, rank, world, dev)
+        train, train_out = measure_train(args, dist, rank, world, dev)
+        if train_out:
+            dump.update(train_out)
 
     if rank == 0:
         resolved = net.resolve_mode()
@@ -589,6 +643,8 @@ def main():
                             'config': {'shard': 'cases', 'note': 'every rank segments its own 512x512x400 volume; no data-path collective'}}
         if train is not None:
             line['train'] = train
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()

@@ -97,7 +97,7 @@ def test_conv_simt_fp32_matches_torch(lib, case):
     L = lib
     mname, Cin, Cout, N, D, H, W = case
     mode = getattr(L, 'CONV_' + mname)
-    g = torch.Generator().manual_seed(hash(case) % 1000)
+    g = torch.Generator().manual_seed(CONV_CASES.index(case))
     x = torch.randn((N, Cin, D, H, W), generator=g)
     wshape = (Cin, Cout, 2, 2, 2) if mode == L.CONV_T2S2 else (Cout, Cin) + {L.CONV_K3: (3, 3, 3), L.CONV_K2S2: (2, 2, 2), L.CONV_K1: (1, 1, 1)}[mode]
     w = torch.randn(wshape, generator=g) * 0.1
@@ -107,7 +107,9 @@ def test_conv_simt_fp32_matches_torch(lib, case):
     assert y.shape == ref.shape
     assert not torch.isnan(y).any()
     assert (y - ref).abs().max() <= 2e-5 * max(1.0, ref.abs().max())        # fp32 FFMA, different summation order
-    s_ref = torch.stack([ref.double().flatten(1).sum(1), (ref.double() ** 2).flatten(1).sum(1)], 1)
+    # the statistics sum the fp32 values the kernel stores: over thousands of voxels the per-voxel rounding differences
+    # from torch add up beyond these bounds, so the sums are taken over the kernel's own output
+    s_ref = torch.stack([y.double().flatten(1).sum(1), (y.double() ** 2).flatten(1).sum(1)], 1)
     assert torch.allclose(stats, s_ref, rtol=1e-5, atol=1e-4)
 
 

@@ -14,6 +14,17 @@ from oracle import sliding_window as osw
 from oracle.metrics import cal_dsc
 
 G = os.path.join(os.path.dirname(__file__), 'golden')
+GOLDEN_THREADS = 8              # tests/golden/make_golden.py computes every fixture with torch.set_num_threads(8)
+
+
+@pytest.fixture(autouse=True)
+def golden_threads():
+    """oneDNN divides a CPU convolution among the threads, and the division sets the fp32 summation order: the oracle
+    reproduces the fixtures to the last bits only with the thread count that computed them, whatever the host's count."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 def seeded_input(seed, shape, kind='noise'):
