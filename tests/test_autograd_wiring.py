@@ -38,9 +38,9 @@ def _install(monkeypatch, calls):
         gd = gamma.t.double().view(1, 1, C)
         if out is None:         # ReLU mask recomputed from the raw tensor: fma(y, rstd*gamma, beta - mean*rstd*gamma) > 0
             assert beta is not None and dres is None
-            a = (rstd.float() * gamma.t.float().view(1, 1, C))
-            z = yv.float() * a + (beta.t.float().view(1, 1, C) - mean.float() * a)
-            dz = g.view(N, nvox, C) * (z > 0)
+            a = (rstd.float() * gamma.t.float().view(1, 1, C)).double()
+            b = (beta.t.double().view(1, 1, C) - mean.float().double() * a).float().double()     # one rounding, like the kernel's FFMA
+            dz = g.view(N, nvox, C) * ((yv * a + b) > 0)
         else:
             dz = (g * (_rows(out, N * nvox, out_ld, C).double() > 0)).view(N, nvox, C)
         if ps == 0:
@@ -166,7 +166,32 @@ def _install(monkeypatch, calls):
         calls.append('adam_step')
         return 0
 
-    table.update({'seg3d_adam_step': adam_step})
+    def _ce_terms(x, t, B, C, n, w, ignore_index):
+        xs = x.t.float().reshape(B, C, n).double()
+        tt = t.t.float().reshape(B, n).long()
+        valid = tt != ignore_index
+        tc = tt.clamp(0, C - 1)
+        wt = (w.t.double().reshape(-1)[tc] if w is not None else torch.ones_like(xs[:, 0])) * valid
+        return xs, tc, wt
+
+    def ce_fwd(x, t, B, C, n, w, ignore_index, part, lmap, stream):
+        xs, tc, wt = _ce_terms(x, t, B, C, n, w, ignore_index)
+        loss = wt * (torch.logsumexp(xs, 1) - xs.gather(1, tc.unsqueeze(1))[:, 0])
+        part.t[0] += loss.sum()
+        part.t[1] += wt.sum()
+        if lmap is not None:
+            lmap.t.copy_(loss.reshape(lmap.t.shape).float())
+        return 0
+
+    def ce_bwd(x, t, B, C, n, w, ignore_index, scale, gmap, grad, stream):
+        xs, tc, wt = _ce_terms(x, t, B, C, n, w, ignore_index)
+        g = torch.softmax(xs, 1)
+        g.scatter_add_(1, tc.unsqueeze(1), -torch.ones_like(xs[:, :1]))
+        g = g * (wt * (gmap.t.double().reshape(B, n) if gmap is not None else scale)).unsqueeze(1)
+        grad.t.copy_(g.reshape(grad.t.shape).float())
+        return 0
+
+    table.update({'seg3d_adam_step': adam_step, 'seg3d_ce_fwd': ce_fwd, 'seg3d_ce_bwd': ce_bwd})
     table.update({'seg3d_gn_bwd': gn_bwd, 'seg3d_conv3d_wgrad': wgrad, 'seg3d_conv3d_cin1_wgrad': cin1_wgrad, 'seg3d_outblock_tail_bwd': tail_bwd,
                   'seg3d_dice_terms': dice_terms, 'seg3d_dice_bwd': dice_bwd, 'seg3d_focal_fwd': focal_fwd, 'seg3d_focal_bwd': focal_bwd})
     monkeypatch.setattr(lib, 'call', lambda name, *a: table[name](*a) if name in table else fwd_call(name, *a))

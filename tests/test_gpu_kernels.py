@@ -386,16 +386,22 @@ WG_CASES = [
     ('K3', 64, 32, 1, 4, 24, 8), ('K3', 16, 32, 2, 5, 16, 16), ('K3', 64, 16, 1, 4, 16, 8), ('K3', 32, 32, 1, 3, 40, 24),   # nine-taps-per-MMA path
     ('K2S2', 32, 64, 2, 8, 32, 16), ('K2S2', 64, 128, 1, 4, 16, 16), ('K2S2', 128, 256, 1, 4, 12, 12),
     ('T2S2', 128, 32, 2, 4, 16, 8), ('T2S2', 256, 64, 1, 2, 12, 12), ('T2S2', 256, 128, 1, 2, 6, 6),
+    # x = the upper half of a 2*Cin-wide buffer, as every down conv reads its skip input from the concat buffer
+    ('K2S2', 16, 32, 2, 8, 12, 16, 'upper'), ('K2S2', 64, 128, 1, 8, 8, 8, 'upper'), ('K3', 32, 32, 2, 8, 16, 8, 'upper'),
+    # out_block.conv1 on the tensor cores: Cout padded to 16, only the first 2 / 5 dy channels nonzero
+    ('K3', 32, 16, 2, 8, 16, 8, 'dy2'), ('K3', 32, 16, 1, 6, 24, 16, 'dy5'),
 ]
 
 
 @pytest.mark.parametrize('dt_name', ['F32', 'BF16'])
 @pytest.mark.parametrize('case', WG_CASES, ids=lambda c: '-'.join(map(str, c)))
 def test_conv_wgrad_matches_torch(lib, case, dt_name):
+    """seg3d_conv3d_wgrad against float64 autograd: |got - ref| <= 2e-5 sum |x| |dy| per weight (fp32 accumulation)"""
     L = lib
     dt = getattr(L, dt_name)
     tdt = L.TORCH_DTYPE[dt]
-    mname, Cin, Cout, N, D, H, W = case
+    mname, Cin, Cout, N, D, H, W = case[:7]
+    variant = case[7] if len(case) > 7 else ''
     mode = getattr(L, 'CONV_' + mname)
     g = torch.Generator().manual_seed(Cin + 5 * Cout)
     x = torch.randn((N, Cin, D, H, W), generator=g).to(tdt).float()
@@ -406,22 +412,35 @@ def test_conv_wgrad_matches_torch(lib, case, dt_name):
     else:
         wshape, od = (Cout, Cin, 3, 3, 3), (D, H, W)
     dy = torch.randn((N, Cout) + od, generator=g).to(tdt).float()
+    if variant.startswith('dy'):
+        dy[:, int(variant[2:]):] = 0
     w = torch.zeros(wshape, dtype=torch.float64, requires_grad=True)
     y = ref_conv(mode, L, x.double(), w, None)
     (y * dy.double()).sum().backward()
-    ref = w.grad.float()
+    ref = w.grad
+    wa = torch.zeros(wshape, dtype=torch.float64, requires_grad=True)
+    ya = ref_conv(mode, L, x.double().abs(), wa, None)
+    (ya * dy.double().abs()).sum().backward()
+    mag = wa.grad
     xd, dyd = to_ndhwc(x, tdt), to_ndhwc(dy, tdt)
+    x_ld, x_off = Cin, 0
+    if variant == 'upper':
+        wide = (torch.randn(xd.shape[:-1] + (2 * Cin,), generator=g) * 1e3).to(tdt).cuda()      # the lower half must not be read
+        wide[..., Cin:] = xd
+        xd, x_ld, x_off = wide, 2 * Cin, Cin
     taps = 27 if mode == L.CONV_K3 else 8
     dw = torch.zeros((taps * Cin * Cout,), dtype=torch.float32, device='cuda')
-    L.call('seg3d_conv3d_wgrad', mode, dt, L.ptr(xd), Cin, Cin, L.ptr(dyd), Cout, Cout, L.ptr(dw), N, D, H, W, L.stream_ptr())
+    L.call('seg3d_conv3d_wgrad', mode, dt, L.ptr(xd, x_off), x_ld, Cin, L.ptr(dyd), Cout, Cout, L.ptr(dw), N, D, H, W, L.stream_ptr())
     torch.cuda.synchronize()
     if mode == L.CONV_T2S2:
         got = dw.view(Cin, 2, 2, 2, Cout).permute(0, 4, 1, 2, 3).cpu()
     else:
         k = 3 if mode == L.CONV_K3 else 2
         got = dw.view(k, k, k, Cin, Cout).permute(4, 3, 0, 1, 2).cpu()
-    err = (got - ref).abs().max() / (ref.abs().max() + 1e-12)
-    assert err <= 2e-3, float(err)
+    err = (got.double() - ref).abs()
+    assert bool((err <= 2e-5 * mag).all()), float((err / (mag + 1e-300)).max())
+    if variant.startswith('dy'):
+        assert bool((got[int(variant[2:]):] == 0).all()), 'gradient of an all-zero dy channel'
 
 
 def test_forward_batch_equals_single(lib):
