@@ -22,13 +22,13 @@ import torch
 import torch.nn.functional as F
 
 from oracle import init as oinit
+from f64_stage_ref import EPS32, _affine32, _close, _mean_rstd32, _rows, _taps, _window  # noqa: F401
 
 pytestmark = pytest.mark.gpu
 
 BF16_REL = 2.0 ** -8        # half an ulp of bf16 (8 significant bits)
 BF16_MAG = 1e-5             # fp32 arithmetic in front of the bf16 store
 F32_MAG = 2e-5              # fp32 accumulation of a parameter gradient, relative to the sum of magnitudes
-EPS32 = float(torch.tensor(1e-5, dtype=torch.float32))      # GN_EPS as the kernels receive it
 
 # arch, classes, loss, B, D, H, W
 CASES = [('vnet', 2, 'dice', 2, 32, 32, 32),
@@ -53,20 +53,6 @@ VNET_CONSUMERS = {
 
 
 # ---- comparison helpers ---------------------------------------------------------------------------------------------
-def _close(name, got, ref, mag, rel, frac):
-    """|got - ref| <= rel |ref| + frac mag elementwise (NaN fails)"""
-    got = got.double()
-    err = (got - ref).abs()
-    tol = rel * ref.abs() + frac * mag
-    bad = ~(err <= tol)
-    if bool(bad.any()):
-        excess = torch.where(bad, (err - tol) / (mag + ref.abs() + 1e-300), torch.zeros_like(err))
-        i = int(torch.argmax(excess.flatten()))
-        raise AssertionError('%s: %d of %d elements out of bound; worst at flat index %d: got %.6g ref %.6g mag %.6g (tol %.3g)'
-                             % (name, int(bad.sum()), bad.numel(), i, float(got.flatten()[i]), float(ref.flatten()[i]),
-                                float(mag.flatten()[i]), float(tol.flatten()[i])))
-
-
 def check_bf16(name, got, ref, mag):
     _close(name, got, ref, mag, BF16_REL, BF16_MAG)
 
@@ -146,35 +132,6 @@ def wgrad_bound(r, u):
     return max(F32_MAG, (S + P) * 2.0 ** -23)
 
 
-def _rows(v, nvox):
-    """[B, nvox, C] float64 copy of the channel window (off, C) of an NDHWC buffer with pitch ld; samples are nvox * ld
-    elements apart, as the kernels address them (a buffer may be allocated wider than the view uses)"""
-    b = v.buf
-    assert v.off + (b.shape[0] * nvox - 1) * v.ld + v.C <= b.numel(), 'view runs past its buffer'
-    return torch.as_strided(b, (b.shape[0], nvox, v.C), (nvox * v.ld, v.ld, 1), b.storage_offset() + v.off).double()
-
-
-def _window(v, off, C):
-    from segmentation3d._b200.plan import _View
-    return _View(v.buf, v.off + off, v.ld, C)
-
-
-def _mean_rstd32(stats, cnt):
-    """gn_mean_rstd (csrc/common.cuh): float64 moments, fp32 mean and rstd; [B, 1, 1] float64 holding fp32 values"""
-    st = stats.double()
-    m = st[:, 0] / cnt
-    var = (st[:, 1] / cnt - m * m).clamp_min(0.0)
-    rstd = 1.0 / torch.sqrt(var + EPS32)
-    return m.float().double().view(-1, 1, 1), rstd.float().double().view(-1, 1, 1)
-
-
-def _affine32(mean, rstd, gamma, beta):
-    """a = fl(rstd * gamma), b = fl(beta - mean * a) with one rounding (FFMA), as the kernels form the ReLU argument"""
-    a = (rstd.float() * gamma.float().view(1, 1, -1)).double()
-    b = (beta.double().view(1, 1, -1) - mean * a).float().double()
-    return a, b
-
-
 def gn_reference(gs, y, stats, gamma, beta, out=None):
     """GroupNorm(1, C) + ReLU (+ residual) backward in float64.  gs: list of [B, nvox, C] gradient contributions, y: raw
     conv output as stored, out: stored activation (its sign is the mask when a residual was added), else the mask is
@@ -205,10 +162,6 @@ def gn_reference(gs, y, stats, gamma, beta, out=None):
     r['dy_mag'] = rstd * (gam.abs() * dz_abs + a1.view(-1, 1, 1) + xh_abs * a2.view(-1, 1, 1))
     r['dbias'], r['dbias_mag'] = r['dy'].sum((0, 1)), r['dy_mag'].sum((0, 1))
     return r
-
-
-def _taps(k):
-    return [(a, b, c) for a in range(k) for b in range(k) for c in range(k)]
 
 
 def wgrad_reference(mode, x, gy):
