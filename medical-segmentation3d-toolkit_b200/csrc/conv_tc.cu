@@ -389,7 +389,9 @@ conv3d_k3_zmarch_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
       constexpr uint32_t ROWB = KC * 2;
       const uint32_t hi_a = desc_hi(p.a_sbo, p.layout_type), hi_b = desc_hi(p.sbo, p.layout_type);
       const uint32_t slab16 = (uint32_t)p.w_slab >> 4, w16 = w_base >> 4;
-      const int nb = p.nb;
+      // nb is 4 or 8: accumulator slot and phase by mask and shift - an integer division by the runtime nb costs ~20
+      // instructions, and this warp's instruction path is the critical path of the plane step (DESIGN.md section 4, finding 9)
+      const int nbm = p.nb - 1, nbs = __ffs(p.nb) - 1;
       for (int item = blockIdx.x; item < p.nitems; item += gridDim.x) {
         const int seg = item % p.nseg;
         const int zs = seg * p.lseg;
@@ -401,20 +403,20 @@ conv3d_k3_zmarch_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
           const int kd_hi = ip < 2 ? ip : 2;                      // kd with 0 <= ip - kd < L
           const int kd_lo = ip - (L - 1) > 0 ? ip - (L - 1) : 0;
           const bool fresh = kd_lo == 0;                          // output plane ip receives its first contribution
-          if (fresh) { const int ocz = oc + ip; mbar_wait(tempty_bar + 8 * (ocz % nb), ((ocz / nb) & 1) ^ 1); tc_fence_after(); }
+          if (fresh) { const int ocz = oc + ip; mbar_wait(tempty_bar + 8 * (ocz & nbm), ((ocz >> nbs) & 1) ^ 1); tc_fence_after(); }
           // runs of adjacent accumulators (planes ip-kd for kd = hi..lo ascend; a run ends at the ring wrap or at maxblk)
           uint32_t dA = 0, bA = 0, iA = 0, dB = 0, bB = 0, iB = 0, dC = 0, bC = 0, iC = 0; int nruns = 0;
           for (int kd = kd_hi; kd >= kd_lo;) {
-            const int b0 = (oc + ip - kd) % nb;
+            const int b0 = (oc + ip - kd) & nbm;
             int len = 1;
-            while (kd - len >= kd_lo && b0 + len < nb && len < p.maxblk) ++len;
+            while (kd - len >= kd_lo && b0 + len <= nbm && len < p.maxblk) ++len;
             const uint32_t d = tmem_base + (uint32_t)(b0 * p.acc_cols), bo = (uint32_t)(2 - kd) * slab16, id = p.idesc0 | ((uint32_t)len * p.n8) << 17;
             if (nruns == 0) { dA = d; bA = bo; iA = id; } else if (nruns == 1) { dB = d; bB = bo; iB = id; } else { dC = d; bC = bo; iC = id; }
             ++nruns;
             kd -= len;
           }
           // the very first MMA into a fresh plane must overwrite: that plane (kd = 0, the last block) is issued on its own
-          const uint32_t dF = tmem_base + (uint32_t)(((oc + ip) % nb) * p.acc_cols);
+          const uint32_t dF = tmem_base + (uint32_t)(((oc + ip) & nbm) * p.acc_cols);
           const uint32_t id1 = p.idesc0 | (p.n8 << 17);
 #pragma unroll
           for (int kh = 0; kh < 3; ++kh)
@@ -430,7 +432,7 @@ conv3d_k3_zmarch_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
                 if (kh == 0 && kw == 0 && k == 0 && fresh) {
                   tc_mma_f16_e(dF, desc_pack(hi_a, da), desc_pack(hi_b, db + 2 * slab16), id1, 0);
                   for (int kd = kd_hi; kd >= 1; --kd)
-                    tc_mma_f16_e(tmem_base + (uint32_t)(((oc + ip - kd) % nb) * p.acc_cols), desc_pack(hi_a, da),
+                    tc_mma_f16_e(tmem_base + (uint32_t)(((oc + ip - kd) & nbm) * p.acc_cols), desc_pack(hi_a, da),
                                desc_pack(hi_b, db + (uint32_t)(2 - kd) * slab16), id1, 1);
                 } else {
                   tc_mma_f16_e(dA, desc_pack(hi_a, da), desc_pack(hi_b, db + bA), iA, 1);
@@ -439,7 +441,7 @@ conv3d_k3_zmarch_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
                 }
               }
           tc_commit_e(empty_bar + 8 * stage);
-          if (ip >= 2) tc_commit_e(tfull_bar + 8 * ((oc + ip - 2) % nb));
+          if (ip >= 2) tc_commit_e(tfull_bar + 8 * ((oc + ip - 2) & nbm));
           if (++stage == p.ring) { stage = 0; phase ^= 1; }
         }
         oc += L;
@@ -519,11 +521,11 @@ conv3d_k3_zmarch_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
       const int gx = x0 + lx, gy = y0 + ly;
       const bool valid = (gx < p.W) && (gy < p.H);
       for (int zl = 0; zl < L; ++zl) {
-        const int ocz = oc + zl, buf = ocz % p.nb;
+        const int ocz = oc + zl, buf = ocz & (p.nb - 1);           // nb is 4 or 8
         const size_t vox = (((size_t)n * p.D + (zs + zl)) * p.H + gy) * p.W + gx;
         T* yrow = y + vox * p.y_ld;
         float* yrow32 = reinterpret_cast<float*>(y) + vox * p.y_ld;
-        mbar_wait(tfull_bar + 8 * buf, (ocz / p.nb) & 1);
+        mbar_wait(tfull_bar + 8 * buf, (ocz >> (__ffs(p.nb) - 1)) & 1);
         tc_fence_after();
         const uint32_t tcol = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * p.acc_cols);
         for (int c0 = half * 16; c0 < p.Cout; c0 += 32) {
