@@ -36,7 +36,8 @@ typedef enum { SEG3D_OK = 0, SEG3D_EINVAL = -1, SEG3D_ECUDA = -2, SEG3D_EUNSUPPO
 typedef enum { SEG3D_F32 = 0, SEG3D_F16 = 1, SEG3D_BF16 = 2 } seg3d_dtype;
 /* OR-ed into `dtype` of seg3d_conv3d_fwd: operands stay f16/bf16 but the raw result y is stored as fp32
  * (pitch y_ld in fp32 elements; y_ld < Cout keeps only the first y_ld channels - used to drop zero-padded output
- * channels).  Tensor-core z-march path only (k3, Cin in {16,32,64}, W % 8 == 0). */
+ * channels).  k3 on the tensor cores: the z-march kernel (Cin in {16,32,64}, W % 8 == 0, weights <= 112 KB), else the
+ * generic kernel, which stores all Cout channels (needs y_ld >= Cout, y_ld % 4 == 0). */
 #define SEG3D_OUT_F32 0x100
 typedef enum {
   SEG3D_CONV_K3 = 0,   /* k=3 s=1 p=1   nn.Conv3d          conv_gn_relu3.py:10, vnet_inblock.py:9, vnet_outblock.py:13 */
@@ -174,6 +175,15 @@ int seg3d_outblock_tail_probs(int dtype, const void* y1, int ld, int C,
                               const float* w2, const float* bias2,
                               const double* stats2, const float* gamma2, const float* beta2, float eps,
                               float* probs, int N, int64_t nvox, void* stream);
+/* The same tail for 1 <= C <= 127 classes on the tensor cores (csrc/tail_wide.cu): the 1x1x1 conv runs as split-operand
+ * f16 MMAs (h = hi + lo, w2 = whi + wlo; hi*whi + lo*whi + hi*wlo into an fp32 accumulator).  y1 is the fp32 raw conv1
+ * result [N][nvox][ld] (16-byte aligned, ld >= C, ld % 4 == 0; channels >= C are never read).  pass 0 accumulates the
+ * GN2 sums into stats2 (caller zeroes); pass 1 reads them and writes probs[n][c][vox] (gamma2, beta2, probs unused in
+ * pass 0).  C outside 1..127 (the int8 label mask) or a misaligned y1 / ld: SEG3D_EUNSUPPORTED. */
+int seg3d_outblock_tail_wide(int pass, const float* y1, int ld, int C,
+                             const double* stats1, const float* gamma1, const float* beta1,
+                             const float* w2, const float* bias2, float eps, double* stats2,
+                             const float* gamma2, const float* beta2, float* probs, int N, int64_t nvox, void* stream);
 
 /* ---- sliding window (core/seg_infer.py:208-246,313-339; utils/image_tools.py:221-238,435-469) -
  * Volumes are fp32 [Z][Y][X] (the reference's numpy order); voxel coordinates are (x,y,z) int32

@@ -887,7 +887,8 @@ int seg3d_conv_tc_supported(int mode, int dtype, int Cin, int Cout, int x_ld, in
   if (dtype != SEG3D_F16 && dtype != SEG3D_BF16) return 0;
   if (Cin % 16 || Cout % 16 || Cout > 256 || Cin > 1024) return 0;
   if (x_ld % 8 || (!out_f32 && y_ld % 8)) return 0;
-  if (out_f32 && !(mode == SEG3D_CONV_K3 && (Cin == 16 || Cin == 32 || Cin == 64) && W % 8 == 0 && D >= 4)) return 0;
+  // fp32 result: the z-march kernel for Cin 16/32/64 (first y_ld channels kept), otherwise the generic kernel's padded fp32 rows
+  if (out_f32 && !(mode == SEG3D_CONV_K3 && (((Cin == 16 || Cin == 32 || Cin == 64) && W % 8 == 0 && D >= 4) || (y_ld >= Cout && y_ld % 4 == 0)))) return 0;
   if (mode == SEG3D_CONV_K2S2 && (D % 2 || H % 2 || W % 2)) return 0;
   return 1;
 }
@@ -1012,7 +1013,11 @@ int seg3d_conv_tc(int mode, int dtype, const void* x, int x_ld, int Cin, const v
   }
   if (xf_nch > 0) { seg3d_set_error("conv_tc: the input transform is only available on the z-march k3 path (Cin 32, W %% 8 == 0, D >= 4)"); return SEG3D_EUNSUPPORTED; }
 
-  SEG3D_REQUIRE(!out_f32, "conv_tc: SEG3D_OUT_F32 (dense real channels) is only available on the z-march k3 path");
+  if (out_f32) {            // the shape did not fit the z-march kernel: all Cout channels as fp32 rows (the strict mode's epilogue)
+    SEG3D_REQUIRE(mode == SEG3D_CONV_K3 && y_ld >= Cout && y_ld % 4 == 0,
+                  "conv_tc: SEG3D_OUT_F32 off the z-march path needs a k3 conv and a pitch y_ld >= Cout that is a multiple of 4");
+    out_f32_generic = 1;
+  }
   TcParams p;
   memset(&p, 0, sizeof(p));
   p.conv = mode == SEG3D_CONV_K2S2 ? 1 : (mode == SEG3D_CONV_T2S2 ? 2 : 0);

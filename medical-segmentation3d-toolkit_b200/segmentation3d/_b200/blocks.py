@@ -15,7 +15,7 @@ import os
 import torch
 
 from . import lib
-from .plan import DEFAULT_TC_MODES, GN_EPS, MODES, _Conv
+from .plan import DEFAULT_TC_MODES, GN_EPS, MODES, WIDE_MAX_CLASSES, _Conv
 
 
 def block_mode(module):
@@ -111,11 +111,10 @@ def conv_gn(x_nd, conv_holder, gn_holder, conv_mode, dt, relu, res=None, out=Non
 
 def output_tail(x_nd, conv1, gn1, conv2, gn2, dt):
     """vnet_outblock.py:20-24: conv1 -> GN1 -> ReLU -> 1x1x1 conv2 -> GN2 -> softmax; fp32 [B,C,D,H,W] probabilities."""
-    B, D, H, W, _ = x_nd.shape
+    B, D, H, W, cin = x_nd.shape
     nc = conv1.weight.shape[0]
-    if nc > 8:
-        raise RuntimeError('seg3d_b200: at most 8 output classes are supported by the out-block tail')
-    raw, s1, c1 = conv_raw(x_nd, conv1, lib.CONV_K3, dt, pad_cout=16)
+    if nc > WIDE_MAX_CLASSES:
+        raise RuntimeError('seg3d_b200: at most %d output classes are supported: the label mask is int8' % WIDE_MAX_CLASSES)
     s2 = torch.zeros((B, 2), dtype=torch.float64, device=x_nd.device)
     g1w, g1b = gn1.weight.detach().float().contiguous(), gn1.bias.detach().float().contiguous()
     g2w, g2b = gn2.weight.detach().float().contiguous(), gn2.bias.detach().float().contiguous()
@@ -123,6 +122,23 @@ def output_tail(x_nd, conv1, gn1, conv2, gn2, dt):
     b2 = conv2.bias.detach().float().contiguous()
     probs = torch.empty((B, nc, D, H, W), dtype=torch.float32, device=x_nd.device)
     nvox = D * H * W
+    if nc > 16:
+        # the whole-network plan's wide path: conv1 zero-padded to Cp channels, its raw result in fp32 rows of pitch Cp, then
+        # the tensor-core tail (csrc/tail_wide.cu)
+        cp = (nc + 15) // 16 * 16
+        c1 = packed_conv(conv1, lib.CONV_K3, dt, pad_cout=cp)
+        if c1.cin != cin:
+            raise ValueError('convolution expects %d input channels, got %d' % (c1.cin, cin))
+        raw = torch.empty((B, D, H, W, cp), dtype=torch.float32, device=x_nd.device)
+        s1 = torch.zeros((B, 2), dtype=torch.float64, device=x_nd.device)
+        with torch.cuda.device(x_nd.device):
+            lib.call('seg3d_conv3d_fwd', c1.mode, dt if dt == lib.F32 else dt | lib.OUT_F32, c1.call_impl, lib.ptr(x_nd), cin, cin,
+                     lib.ptr(c1.w), lib.ptr(c1.bias), lib.ptr(raw), cp, c1.cout, B, D, H, W, lib.ptr(s1), lib.stream_ptr())
+            for ps in (0, 1):
+                lib.call('seg3d_outblock_tail_wide', ps, lib.ptr(raw), cp, nc, lib.ptr(s1), lib.ptr(g1w), lib.ptr(g1b), lib.ptr(w2),
+                         lib.ptr(b2), GN_EPS, lib.ptr(s2), lib.ptr(g2w), lib.ptr(g2b), lib.ptr(probs), B, nvox, lib.stream_ptr())
+        return probs
+    raw, s1, c1 = conv_raw(x_nd, conv1, lib.CONV_K3, dt, pad_cout=16)
     with torch.cuda.device(x_nd.device):
         lib.call('seg3d_outblock_tail_stats', dt, lib.ptr(raw), c1.cout, nc, lib.ptr(s1), lib.ptr(g1w), lib.ptr(g1b), lib.ptr(w2),
                  lib.ptr(b2), GN_EPS, lib.ptr(s2), B, nvox, lib.stream_ptr())

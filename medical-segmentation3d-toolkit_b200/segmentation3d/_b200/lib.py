@@ -42,6 +42,7 @@ _SIGNATURES = {
     'seg3d_gn_apply': (_i, [_i, _vp, _i, _i, _vp, _vp, _vp, _f, _vp, _i, _vp, _i, _i, _i, _i64, _vp]),
     'seg3d_outblock_tail_stats': (_i, [_i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _vp, _i, _i64, _vp]),
     'seg3d_outblock_tail_probs': (_i, [_i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _vp, _i, _i64, _vp]),
+    'seg3d_outblock_tail_wide': (_i, [_i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp, _vp, _i, _i64, _vp]),
     'seg3d_patch_stats': (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i, _i, _vp, _vp]),
     'seg3d_patch_gather': (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _f, _f, _i, _f, _f, _vp, _i, _vp, _vp]),
     'seg3d_patch_gather_rows': (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _f, _f, _i, _f, _f, _vp, _i, _vp, _i, _i, _vp]),

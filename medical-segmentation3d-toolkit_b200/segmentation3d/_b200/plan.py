@@ -186,8 +186,13 @@ class NetPlan(object):
         self.tc_modes = tuple(tc_modes)
         self.in_channels = sd['in_block.conv.weight'].shape[1]
         self.out_channels = sd['out_block.conv2.weight'].shape[0]
-        if self.out_channels > 16:
-            raise RuntimeError('seg3d_b200: at most 16 output classes are supported by the out-block tail kernels')
+        if self.out_channels > WIDE_MAX_CLASSES:
+            raise RuntimeError('seg3d_b200: at most %d output classes are supported: the label mask is int8 '
+                               '(seg3d_blend_finalize_argmax_z)' % WIDE_MAX_CLASSES)
+        # more than 16 classes: the tensor-core tail (csrc/tail_wide.cu) on conv1's raw result, zero-padded to `wide_cp`
+        # output channels and stored in fp32; up to 16 the SIMT tail stays the exact-fp32 path
+        self.wide = self.out_channels > 16
+        self.wide_cp = (self.out_channels + 15) // 16 * 16
         self.convs, self.gns = {}, {}
         for k in sd:
             if not k.endswith('.weight'):
@@ -205,8 +210,9 @@ class NetPlan(object):
                 narrow = (name == 'out_block.conv1' and self.dt != lib.F32 and lib.CONV_K3 in self.tc_modes
                           and sd[k].shape[0] <= 7 and sd[k].shape[1] in ((32,) if self.split else (16, 32, 64))
                           and os.environ.get('SEG3D_NARROW', '1') != '0')
+                pad = (self.wide_cp if self.wide else 16) if name == 'out_block.conv1' else 0
                 self.convs[name] = _Conv(sd, name, m, self.dt, self.device, self.tc_modes,
-                                         pad_cout=16 if name == 'out_block.conv1' else 0, fold=narrow, split=self.split)
+                                         pad_cout=pad, fold=narrow, split=self.split)
             else:
                 self.gns[name] = _GN(sd, name, self.device)
         self.w2 = sd['out_block.conv2.weight'].detach().to(self.device, torch.float32).reshape(
@@ -272,6 +278,9 @@ class NetPlan(object):
         split = self.split
         if split and train:
             raise RuntimeError("seg3d_b200: mode 'fp32x' is an inference mode (train in 'bf16' or 'fp32')")
+        if self.wide and train:
+            raise RuntimeError('seg3d_b200: training supports up to 16 classes (this net has %d); nets with up to %d classes '
+                               'run inference only' % (self.out_channels, WIDE_MAX_CLASSES))
         cm = 2 if split else 1          # split mode: every activation row is [hi(C) | lo(C)]
         dims = [(D >> l, H >> l, W >> l) for l in range(5)]
         vox = [d[0] * d[1] * d[2] for d in dims]
@@ -530,7 +539,20 @@ class NetPlan(object):
         tail_f32 = (c1.impl == lib.IMPL_TCGEN05 and src.C in (16, 32, 64) and W % 8 == 0 and not train and not split
                     and os.environ.get('SEG3D_TAIL_F32', '1') != '0')
         tail_dt = lib.F32 if (tail_f32 or split) else dt
-        if tail_f32 and c1.fold:
+        if self.wide:
+            # raw conv1 result in fp32 rows of pitch wide_cp (a multiple of 4 floats, as the tail's TMA needs) in every mode:
+            # the z-march kernel up to 64 padded channels (32 in fp32x), the generic tensor-core kernel above, SIMT in fp32
+            ncp = self.wide_cp
+            rv1 = _View(torch.empty((B, vox[0], ncp), dtype=torch.float32, device=dev), 0, ncp, c1.cout, sample=vox[0] * ncp)
+            if dt == lib.F32 or split:
+                conv('out_block.conv1', src, dims[0], rv1, 'out_block.gn1', 0)
+            else:
+                add(lambda b0, nb: lib.call('seg3d_conv3d_fwd', c1.mode, dt | lib.OUT_F32, c1.impl, src.at(b0), src.ld, c1.cin,
+                                            lib.ptr(c1.w), lib.ptr(c1.bias), rv1.at(b0), rv1.ld, c1.cout, nb, dims[0][0], dims[0][1],
+                                            dims[0][2], stats_ptr('out_block.gn1', b0), st()), 0)
+                meta.append({'name': 'out_block.conv1', 'kind': 'conv_tc_k3', 'flops': 2.0 * B * vox[0] * 27 * c1.cin * c1.cout,
+                             'bytes': 2 * B * vox[0] * c1.cin + 4 * B * vox[0] * c1.cout + c1.w.numel() * 2})
+        elif tail_f32 and c1.fold:
             # nine in-plane taps folded into the GEMM N dimension (csrc/conv_tc_narrow.cu), fp32 result
             ncp = nc
             rv1 = _View(torch.empty((B, vox[0], nc), dtype=torch.float32, device=dev), 0, nc, nc, sample=vox[0] * nc)
@@ -592,6 +614,21 @@ class NetPlan(object):
                      lib.ptr(g1.beta), lib.ptr(self.w2), lib.ptr(self.b2), lib.ptr(ws['stats2'], 2 * b0), lib.ptr(g2.gamma),
                      lib.ptr(g2.beta), GN_EPS, lib.ptr(probs, b0 * psample), nb, vox[0], st())
 
+        if self.wide:
+            def tail_wide(ps):
+                return lambda b0, nb: lib.call('seg3d_outblock_tail_wide', ps, rv1.at(b0), rv1.ld, nc, stats_ptr('out_block.gn1', b0),
+                                               lib.ptr(g1.gamma), lib.ptr(g1.beta), lib.ptr(self.w2), lib.ptr(self.b2), GN_EPS,
+                                               lib.ptr(ws['stats2'], 2 * b0), lib.ptr(g2.gamma), lib.ptr(g2.beta),
+                                               lib.ptr(probs, b0 * psample), nb, vox[0], st())
+            add(tail_wide(0), 0)
+            add(tail_wide(1), 0)
+            # per voxel: 3 * Cp / 16 MMAs of K = 16 on Cp columns; pass 0 reads the raw row, pass 1 reads it and writes C probs
+            flops = 2.0 * 3 * B * vox[0] * ncp * ncp
+            meta.append({'name': 'out_block.tail_stats', 'kind': 'tail_wide', 'flops': flops, 'bytes': 4 * B * vox[0] * ncp})
+            meta.append({'name': 'out_block.tail_probs', 'kind': 'tail_wide', 'flops': flops,
+                         'bytes': 4 * B * vox[0] * ncp + 4 * B * vox[0] * nc})
+            ws['schedule'] = self._schedule(B, levels, vox, train)
+            return ws, ops
         add(tail_stats, 0)
         add(tail_probs, 0)
         esz = 4 if dt == lib.F32 else 2
@@ -717,3 +754,4 @@ class NetPlan(object):
 
 
 DEFAULT_TC_MODES = (lib.CONV_K3, lib.CONV_K2S2, lib.CONV_T2S2)
+WIDE_MAX_CLASSES = 127
