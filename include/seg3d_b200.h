@@ -303,6 +303,24 @@ int seg3d_outblock_tail_bwd(int dtype, int pass, const void* y1, int ld, int C,
                             float* dgamma2, float* dbeta2, float* dw2, float* db2,
                             float* dgamma1, float* dbeta1, float* db1,
                             void* dy1, int dy_ld, int N, int64_t nvox, void* stream);
+/* seg3d_gn_bwd without the ReLU: the backward of a unit that ends in a plain GroupNorm (a standalone
+ * ConvGnRelu3(..., do_act=False)).  Same two passes, arguments and outputs as seg3d_gn_bwd with dz = g0 + g1 + g2
+ * (no mask: there is no `out` and no beta).  dres (optional) = dz.  C % 8 == 0, 256 % (C/8) == 0, pitches % 8 == 0. */
+int seg3d_gn_bwd_noact(int dtype, int pass, const void* g0, int ld0, const void* g1, int ld1, const void* g2, int ld2,
+                       const void* y, int y_ld, int C, const double* stats, const float* gamma, float eps,
+                       double* sums, float* dgamma, float* dbeta, void* dy, int dy_ld, void* dres, int dres_ld,
+                       float* dbias, int N, int64_t nvox, void* stream);
+/* Layout boundary of the standalone modules' backward (NCDHW fp32 outside a module, NDHWC storage type inside).
+ * seg3d_grad_to_ncdhw: out[n][c][v] (fp32, dense [N][C][nvox]) = g0 + g1 + g2 summed in fp32 in that order, where
+ *   contribution k (k < n_contrib, 1..3) is the NDHWC window gk[(n*nvox + v)*ldk + offk + c], c < C, in the storage type
+ *   `dtype` (ldk >= offk + C).  Unused contributions may be NULL.
+ * seg3d_grad_from_ncdhw: out[(n*nvox + v)*ld + off + c] = in[n][c][v] rounded to the storage type; channels outside
+ *   [off, off + C) of each row are not written.
+ * 16-byte accesses on the NDHWC side need C, pitch and offset multiples of 16 / sizeof(storage type) and a 16-byte
+ * aligned base; other layouts take a scalar path. */
+int seg3d_grad_to_ncdhw(int dtype, int n_contrib, const void* g0, int ld0, int off0, const void* g1, int ld1, int off1,
+                        const void* g2, int ld2, int off2, int C, int N, int64_t nvox, float* out, void* stream);
+int seg3d_grad_from_ncdhw(int dtype, const float* in, int C, int N, int64_t nvox, void* out, int ld, int off, void* stream);
 
 /* ---- training: the parameter side of the step (reference core/seg_train.py:83 `optim.Adam(net.parameters(), lr, betas)`,
  * :127 `opt.step()`; the per-step weight re-layout replaces what nn.Conv3d does implicitly by reading its own parameter) ----

@@ -14,6 +14,8 @@
 // the forward apply evaluated on the same stored y, so `out` is not read at all - a third of pass 0's traffic)
 //     dy = rstd*(gamma*dz - mean_all(gamma*dz) - xhat*mean_all(gamma*dz*xhat)),
 //     dgamma_c = sum dz*xhat, dbeta_c = sum dz, dres = dz, dbias_c = sum dy.
+// A unit without the ReLU (a standalone ConvGnRelu3(..., do_act=False) ends in a plain GroupNorm) takes the same two passes
+// with dz = g (NOACT: no mask, neither `out` nor beta read).
 #include "common.cuh"
 
 namespace {
@@ -23,7 +25,7 @@ constexpr int GN_BWD_U = 4;
 
 // PASS 0: per-sample sums S1 = sum gamma*dz, S2 = sum gamma*dz*xhat; per-channel dgamma, dbeta.
 // PASS 1: dy (+ optional dres), per-channel dbias.
-template <typename T, int PASS, bool REMASK>
+template <typename T, int PASS, bool REMASK, bool NOACT = false>
 __global__ void __launch_bounds__(256, 2)
 gn_bwd_kernel(const T* __restrict__ g0, int ld0, const T* __restrict__ g1, int ld1, const T* __restrict__ g2, int ld2,
               const T* __restrict__ out, int out_ld, const T* __restrict__ y, int y_ld, int C,
@@ -69,7 +71,7 @@ gn_bwd_kernel(const T* __restrict__ g0, int ld0, const T* __restrict__ g1, int l
       rg0[u].load(g0 + vv * ld0 + c0);
       if (g1) rg1[u].load(g1 + vv * ld1 + c0); else rg1[u].zero();
       if (g2) rg2[u].load(g2 + vv * ld2 + c0); else rg2[u].zero();
-      if (!REMASK) ro[u].load(out + vv * out_ld + c0);
+      if (!REMASK && !NOACT) ro[u].load(out + vv * out_ld + c0);
       ry[u].load(y + vv * y_ld + c0);
     }
 #pragma unroll
@@ -79,11 +81,11 @@ gn_bwd_kernel(const T* __restrict__ g0, int ld0, const T* __restrict__ g1, int l
       const size_t vv = nb + vu;
       float ga[8], gb[8], gc[8], o[8], yy[8];
       rg0[u].get(ga); rg1[u].get(gb); rg2[u].get(gc); ry[u].get(yy);
-      if (!REMASK) ro[u].get(o);
+      if (!REMASK && !NOACT) ro[u].get(o);
       float dyv[8], dzv[8];
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
-        const bool on = REMASK ? (fmaf(yy[j], za[j], zb[j]) > 0.f) : (o[j] > 0.f);
+        const bool on = NOACT || (REMASK ? (fmaf(yy[j], za[j], zb[j]) > 0.f) : (o[j] > 0.f));
         const float dz = on ? (ga[j] + gb[j] + gc[j]) : 0.f;
         const float xh = (yy[j] - mean) * rstd;
         if (PASS == 0) {
@@ -477,6 +479,32 @@ extern "C" int seg3d_gn_bwd(int dtype, int pass, const void* g0, int ld0, const 
   SEG3D_DISPATCH_DTYPE(dtype, T, {
     if (pass == 0) { if (out) SEG3D_GNB(0, false); else SEG3D_GNB(0, true); }
     else           { if (out) SEG3D_GNB(1, false); else SEG3D_GNB(1, true); }
+  });
+#undef SEG3D_GNB
+  SEG3D_CHECK_LAUNCH("gn_bwd_kernel");
+  return SEG3D_OK;
+}
+
+extern "C" int seg3d_gn_bwd_noact(int dtype, int pass, const void* g0, int ld0, const void* g1, int ld1, const void* g2, int ld2,
+                                  const void* y, int y_ld, int C, const double* stats, const float* gamma, float eps,
+                                  double* sums, float* dgamma, float* dbeta, void* dy, int dy_ld, void* dres, int dres_ld,
+                                  float* dbias, int N, int64_t nvox, void* stream) {
+  SEG3D_REQUIRE(C > 0 && C % 8 == 0 && C <= GN_BWD_MAXC && 256 % (C / 8) == 0, "gn_bwd_noact: unsupported C=%d", C);
+  SEG3D_REQUIRE(g0 && y && stats && gamma && sums && N > 0 && nvox > 0, "gn_bwd_noact: bad arguments");
+  SEG3D_REQUIRE(pass == 0 ? (dgamma && dbeta) : (dy != nullptr), "gn_bwd_noact: missing outputs for pass %d", pass);
+  SEG3D_REQUIRE(ld0 % 8 == 0 && (!g1 || ld1 % 8 == 0) && (!g2 || ld2 % 8 == 0) && y_ld % 8 == 0,
+                "gn_bwd_noact: pitches must be multiples of 8");
+  SEG3D_REQUIRE(pass == 0 || (dy_ld % 8 == 0 && (!dres || dres_ld % 8 == 0)), "gn_bwd_noact: pitches must be multiples of 8");
+  const int cv = C / 8, vpb = 256 / cv;
+  long long want = (nvox + vpb * 4 - 1) / (vpb * 4);
+  const int sms = seg3d_num_sms();
+  int gx = (int)(want < 1 ? 1 : (want > 4LL * sms ? 4LL * sms : want));
+  dim3 grid(gx, N);
+  cudaStream_t st = (cudaStream_t)stream;
+#define SEG3D_GNB(PS) gn_bwd_kernel<T, PS, false, true><<<grid, 256, 0, st>>>((const T*)g0, ld0, (const T*)g1, ld1, (const T*)g2, ld2, \
+        (const T*)nullptr, 0, (const T*)y, y_ld, C, stats, gamma, nullptr, eps, sums, dgamma, dbeta, (T*)dy, dy_ld, (T*)dres, dres_ld, dbias, nvox)
+  SEG3D_DISPATCH_DTYPE(dtype, T, {
+    if (pass == 0) SEG3D_GNB(0); else SEG3D_GNB(1);
   });
 #undef SEG3D_GNB
   SEG3D_CHECK_LAUNCH("gn_bwd_kernel");

@@ -33,6 +33,38 @@ _k3_dgrad_weight.seg3d_kind = 'k3_dgrad'       # index-map forms of these transf
 _same_weight.seg3d_kind = 'identity'
 
 
+def unit_step(dt, B, gsrc, out, raw, C, stats, gamma, beta, sums, dgamma, dbeta, gy, dres, dbias, nvox, mode, x, cin, dw, xd,
+              dgrad=None, relu=True, xpad=None):
+    """Backward of one conv -> GroupNorm [-> ReLU] [+ residual] unit, shared by the whole-network walk (_Backward.run) and
+    the standalone modules (blocks.py):
+        gn_bwd pass 0/1   dz = sum of the output's gradient contributions `gsrc` (1..3 _Views), masked by the ReLU when
+                          `relu`; dy -> gy, dz -> dres (a unit with a residual), dgamma/dbeta/dbias
+        conv wgrad        dw (kernel layout, fp32, accumulated) from the unit's input x (dims xd) and gy
+        conv dgrad        dgrad = (dgrad convolution, gradient view, gy's dims), or None when no input gradient is needed
+    `xpad` (whole network only): the input block's row-padded input, whose weight gradient has a kernel of its own."""
+    st = lib.stream_ptr
+    gv = list(gsrc) + [None] * (3 - len(gsrc))
+    g = (gv[0].p, gv[0].ld, gv[1].p if gv[1] else None, gv[1].ld if gv[1] else 0, gv[2].p if gv[2] else None, gv[2].ld if gv[2] else 0)
+    if relu:
+        # without a residual the ReLU mask is recomputed from the raw tensor the kernel reads anyway (out = NULL)
+        remask = dres is None and os.environ.get('SEG3D_GN_BWD_REMASK', '1') != '0'
+        for p in range(2):
+            lib.call('seg3d_gn_bwd', dt, p, *g, None if remask else out.p, out.ld, raw.p, raw.ld, C, stats, gamma, beta, GN_EPS,
+                     sums, dgamma, dbeta, gy.p, gy.ld, dres.p if dres else None, dres.ld if dres else 0, dbias, B, nvox, st())
+    else:
+        for p in range(2):
+            lib.call('seg3d_gn_bwd_noact', dt, p, *g, raw.p, raw.ld, C, stats, gamma, GN_EPS,
+                     sums, dgamma, dbeta, gy.p, gy.ld, dres.p if dres else None, dres.ld if dres else 0, dbias, B, nvox, st())
+    if xpad is not None:
+        lib.call('seg3d_conv3d_cin1_wgrad', dt, xpad.p, xd[2] + lib.CIN1_PAD, gy.p, gy.ld, dw, B, xd[0], xd[1], xd[2], st())
+    else:
+        lib.call('seg3d_conv3d_wgrad', mode, dt, x.p, x.ld, cin, gy.p, gy.ld, C, dw, B, xd[0], xd[1], xd[2], st())
+    if dgrad is not None:
+        dcv, gd, od = dgrad
+        lib.call('seg3d_conv3d_fwd', dcv.mode, dt, dcv.impl, gy.p, gy.ld, dcv.cin, lib.ptr(dcv.w), None,
+                 gd.p, gd.ld, dcv.cout, B, od[0], od[1], od[2], None, st())
+
+
 class _Backward(object):
     """Per (plan, shape) backward state: gradient buffers, dgrad convolutions, parameter-gradient slots."""
 
@@ -221,37 +253,22 @@ class _Backward(object):
             c = plan.convs[u['conv']]
             gsrc = contrib.get((id(u['out'].buf), u['out'].off), [])
             assert 1 <= len(gsrc) <= 3, (u['conv'], len(gsrc))
-            gv = gsrc + [None] * (3 - len(gsrc))
             gnp = plan.gns[u['gn']]
             sf = lib.ptr(ws['stats'][plan.gn_index[u['gn']]])
             gy = self.gy[u['conv']]
             dres = self.dres.get(u['conv'])
-            nv = vox[u['lout']]
-            # without a residual the ReLU mask is recomputed from the raw tensor the kernel reads anyway (out = NULL)
-            remask = dres is None and os.environ.get('SEG3D_GN_BWD_REMASK', '1') != '0'
-            for p in range(2):
-                lib.call('seg3d_gn_bwd', dt, p, gv[0].p, gv[0].ld, gv[1].p if gv[1] else None, gv[1].ld if gv[1] else 0,
-                         gv[2].p if gv[2] else None, gv[2].ld if gv[2] else 0,
-                         None if remask else u['out'].p, u['out'].ld, u['raw'].p, u['raw'].ld, c.cout, sf, lib.ptr(gnp.gamma),
-                         lib.ptr(gnp.beta), GN_EPS,
-                         lib.ptr(self.sums[ui]), lib.ptr(pg[u['gn'] + '.weight']), lib.ptr(pg[u['gn'] + '.bias']),
-                         gy.p, gy.ld, dres.p if dres else None, dres.ld if dres else 0,
-                         lib.ptr(pg[u['conv'] + '.bias']), B, nv, st())
+            dgrad = None
+            if u['conv'] in self.gd:           # the dgrad convolution's input is dy, living at the unit's output level
+                dgrad = (self.dconv[u['conv']], self.gd[u['conv']], dims[u['lout']])
+            # input block on the row-padded input (Toeplitz operands)
+            xpad = u['xpad'] if u.get('xpad') is not None and gy.ld == 16 else None
+            unit_step(dt, B, gsrc, u['out'], u['raw'], c.cout, sf, lib.ptr(gnp.gamma), lib.ptr(gnp.beta), lib.ptr(self.sums[ui]),
+                      lib.ptr(pg[u['gn'] + '.weight']), lib.ptr(pg[u['gn'] + '.bias']), gy, dres, lib.ptr(pg[u['conv'] + '.bias']),
+                      vox[u['lout']], c.mode, u['x'], c.cin, lib.ptr(pg[u['conv'] + '.weight']), dims[u['lin']], dgrad, xpad=xpad)
             if dres is not None:
                 add_contrib(u['res'], dres)
-            xd = dims[u['lin']]
-            if u.get('xpad') is not None and gy.ld == 16:       # input block on the row-padded input (Toeplitz operands)
-                lib.call('seg3d_conv3d_cin1_wgrad', dt, u['xpad'].p, xd[2] + lib.CIN1_PAD, gy.p, gy.ld,
-                         lib.ptr(pg[u['conv'] + '.weight']), B, xd[0], xd[1], xd[2], st())
-            else:
-                lib.call('seg3d_conv3d_wgrad', c.mode, dt, u['x'].p, u['x'].ld, c.cin, gy.p, gy.ld, c.cout,
-                         lib.ptr(pg[u['conv'] + '.weight']), B, xd[0], xd[1], xd[2], st())
-            if u['conv'] in self.gd:
-                dcv, gd = self.dconv[u['conv']], self.gd[u['conv']]
-                od = dims[u['lout']]          # the dgrad convolution's input is dy, living at the unit's output level
-                lib.call('seg3d_conv3d_fwd', dcv.mode, dt, dcv.impl, gy.p, gy.ld, dcv.cin, lib.ptr(dcv.w), None,
-                         gd.p, gd.ld, dcv.cout, B, od[0], od[1], od[2], None, st())
-                add_contrib(u['x'], gd)
+            if dgrad is not None:
+                add_contrib(u['x'], dgrad[1])
             reduce_tail(self.pg_off[u['conv'] + '.weight'])
         reduce_tail(0, force=True)
         for w in works:

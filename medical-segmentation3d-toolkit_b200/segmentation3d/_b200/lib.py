@@ -61,6 +61,10 @@ _SIGNATURES = {
     'seg3d_ce_bwd': (_i, [_vp, _vp, _i, _i, _i64, _vp, _i, _f, _vp, _vp, _vp]),
     'seg3d_gn_bwd': (_i, [_i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _vp, _f, _vp, _vp, _vp,
                           _vp, _i, _vp, _i, _vp, _i, _i64, _vp]),
+    'seg3d_gn_bwd_noact': (_i, [_i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _f, _vp, _vp, _vp,
+                                _vp, _i, _vp, _i, _vp, _i, _i64, _vp]),
+    'seg3d_grad_to_ncdhw': (_i, [_i, _i, _vp, _i, _i, _vp, _i, _i, _vp, _i, _i, _i, _i, _i64, _vp, _vp]),
+    'seg3d_grad_from_ncdhw': (_i, [_i, _vp, _i, _i, _i64, _vp, _i, _i, _vp]),
     'seg3d_conv3d_wgrad': (_i, [_i, _i, _vp, _i, _i, _vp, _i, _i, _vp, _i, _i, _i, _i, _vp]),
     'seg3d_outblock_tail_bwd': (_i, [_i, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp,
                                      _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i64, _vp]),

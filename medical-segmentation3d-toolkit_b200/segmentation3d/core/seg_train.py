@@ -54,7 +54,15 @@ def make_optimizer(net, lr, betas=(0.9, 0.999)):
     state-dict layout, same update rule - whose step() is one C-ABI launch over all parameters (_b200/optim.py)."""
     from segmentation3d._b200.optim import FlatAdam
     root = getattr(net, 'module', net)
-    return FlatAdam(net.parameters(), lr=lr, betas=betas, on_step=getattr(root, 'mark_weights_changed', None))
+    on_step = getattr(root, 'mark_weights_changed', None)
+    if on_step is None:
+        # a network assembled from the standalone modules re-packs a convolution's weights when the parameter's version
+        # counter moves (blocks.packed_conv); the Adam kernel writes the parameters behind torch's back, so move it here
+        params = list(net.parameters())
+
+        def on_step():
+            torch.autograd.graph.increment_version(params)
+    return FlatAdam(net.parameters(), lr=lr, betas=betas, on_step=on_step)
 
 
 def train_step(net, opt, loss_func, crops, masks, params=None, return_outputs=False):

@@ -10,18 +10,20 @@ from segmentation3d.network.module.conv_gn_relu3 import BottConvGnRelu3, ConvGnR
 class _ResidualBase(nn.Module):
     channels = 0
 
-    def _run(self, x_nd, dt):
+    def _run(self, x_nd, dt, tape=None):
         y = x_nd
         n = len(self.ops)
         for i, op in enumerate(self.ops):
             last = i == n - 1
-            y = op._run(y, dt, res=x_nd if last else None, relu=True)     # last unit: relu(gn(conv) + x)
+            y = op._run(y, dt, res=x_nd if last else None, relu=True, tape=tape)     # last unit: relu(gn(conv) + x)
         return y
+
+    def _forward(self, dt, tape, input):
+        return blocks.to_ncdhw(self._run(blocks.to_ndhwc(input, dt, tape), dt, tape), tape)
 
     def forward(self, input):
         blocks.check_input(input, self.channels)
-        _, dt = blocks.block_mode(self)
-        return blocks.to_ncdhw(self._run(blocks.to_ndhwc(input, dt), dt))
+        return blocks.run_module(self, self._forward, input)
 
 
 class ResidualBlock3(_ResidualBase):

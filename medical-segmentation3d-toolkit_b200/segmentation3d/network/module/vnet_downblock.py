@@ -19,8 +19,10 @@ class DownBlock(nn.Module):
         else:
             self.rblock = ResidualBlock3(out_channels, 3, 1, 1, num_convs)
 
+    def _forward(self, dt, tape, input):
+        out = blocks.conv_gn(blocks.to_ndhwc(input, dt, tape), self.down_conv, self.down_gn, lib.CONV_K2S2, dt, True, tape=tape)
+        return blocks.to_ncdhw(self.rblock._run(out, dt, tape), tape)
+
     def forward(self, input):
         blocks.check_input(input, self.down_conv.in_channels)
-        _, dt = blocks.block_mode(self)
-        out = blocks.conv_gn(blocks.to_ndhwc(input, dt), self.down_conv, self.down_gn, lib.CONV_K2S2, dt, True)
-        return blocks.to_ncdhw(self.rblock._run(out, dt))
+        return blocks.run_module(self, self._forward, input)

@@ -12,7 +12,10 @@ class InputBlock(nn.Module):
         self.gn = GroupNormParams(out_channels)
         self.act = nn.ReLU(inplace=True)
 
+    def _forward(self, dt, tape, input):
+        x = blocks.to_ndhwc(input, dt, tape)
+        return blocks.to_ncdhw(blocks.conv_gn(x, self.conv, self.gn, lib.CONV_K3, dt, True, tape=tape), tape)
+
     def forward(self, input):
         blocks.check_input(input, self.conv.in_channels)
-        _, dt = blocks.block_mode(self)
-        return blocks.to_ncdhw(blocks.conv_gn(blocks.to_ndhwc(input, dt), self.conv, self.gn, lib.CONV_K3, dt, True))
+        return blocks.run_module(self, self._forward, input)

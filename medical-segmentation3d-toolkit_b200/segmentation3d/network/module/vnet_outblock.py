@@ -1,5 +1,6 @@
 """Output block (drop-in for reference network/module/vnet_outblock.py:4-24): conv k3 -> GroupNorm -> ReLU -> conv k1 ->
-GroupNorm -> channel softmax; returns fp32 probabilities [B, classes, D, H, W]."""
+GroupNorm -> channel softmax; returns fp32 probabilities [B, classes, D, H, W].  Trains with up to 16 classes (the
+tail backward of the whole network); wider blocks run inference under torch.no_grad()."""
 import torch.nn as nn
 
 from segmentation3d._b200 import blocks
@@ -16,7 +17,9 @@ class OutputBlock(nn.Module):
         self.gn2 = GroupNormParams(out_channels)
         self.softmax = nn.Softmax(dim=1)
 
+    def _forward(self, dt, tape, input):
+        return blocks.output_tail(blocks.to_ndhwc(input, dt, tape), self.conv1, self.gn1, self.conv2, self.gn2, dt, tape)
+
     def forward(self, input):
         blocks.check_input(input, self.conv1.in_channels)
-        _, dt = blocks.block_mode(self)
-        return blocks.output_tail(blocks.to_ndhwc(input, dt), self.conv1, self.gn1, self.conv2, self.gn2, dt)
+        return blocks.run_module(self, self._forward, input)

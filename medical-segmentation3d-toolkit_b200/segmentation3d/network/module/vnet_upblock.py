@@ -20,16 +20,22 @@ class UpBlock(nn.Module):
         else:
             self.rblock = ResidualBlock3(out_channels, 3, 1, 1, num_convs)
 
-    def forward(self, input, skip):
+    def _forward(self, dt, tape, input, skip):
         half = self.up_conv.out_channels
-        blocks.check_input(input, self.up_conv.in_channels)
-        blocks.check_input(skip, self.rblock.channels - half)
-        _, dt = blocks.block_mode(self)
-        raw, stats, _ = blocks.conv_raw(blocks.to_ndhwc(input, dt), self.up_conv, lib.CONV_T2S2, dt)
+        x = blocks.to_ndhwc(input, dt, tape)
+        raw, stats, conv = blocks.conv_raw(x, self.up_conv, lib.CONV_T2S2, dt)
         B, D, H, W, _ = raw.shape
         if tuple(skip.shape[2:]) != (D, H, W):
             raise ValueError('skip tensor must have the up-sampled spatial size %s, got %s' % ((D, H, W), tuple(skip.shape[2:])))
         cat = torch.empty((B, D, H, W, self.rblock.channels), dtype=raw.dtype, device=raw.device)
         cat[..., half:].copy_(skip.detach().permute(0, 2, 3, 4, 1))          # vnet_upblock.py:21: (up, skip) along channels
         blocks.gn_apply(raw, stats, self.up_gn, dt, True, out=cat, out_off=0)
-        return blocks.to_ncdhw(self.rblock._run(cat, dt))
+        if tape is not None:        # the skip tensor's gradient is the upper channel window of the concat's gradient
+            tape.input(1, blocks._View(cat, half, cat.shape[-1], cat.shape[-1] - half))
+            tape.unit(x, self.up_conv, self.up_gn, lib.CONV_T2S2, conv, raw, stats, cat, 0, True, None)
+        return blocks.to_ncdhw(self.rblock._run(cat, dt, tape), tape)
+
+    def forward(self, input, skip):
+        blocks.check_input(input, self.up_conv.in_channels)
+        blocks.check_input(skip, self.rblock.channels - self.up_conv.out_channels)
+        return blocks.run_module(self, self._forward, input, skip)
