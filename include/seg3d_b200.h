@@ -93,6 +93,13 @@ int seg3d_conv3d_cin1_fwd(int dtype, int epi_mode, const void* xpad, int x_pitch
 int seg3d_conv3d_cin1_wgrad(int dtype, const void* xpad, int x_pitch, const void* dy, int dy_ld, float* dw,
                             int N, int D, int H, int W, void* stream);
 
+/* data gradient of the input block, written as the NCDHW fp32 input gradient: dx[n][0][z][y][x] (dense [N,1,D,H,W]) =
+ * sum over taps (a,b,c) and co < 16 of w[(a*3+b)*3+c][co] * gy[n][z+1-a][y+1-b][x+1-c][co], zero outside the volume,
+ * accumulated in fp32.  gy: [N,D,H,W,16] in `dtype` (f32/f16/bf16) with pitch ld (>= 16, ld * sizeof % 16 == 0);
+ * w: fp32 [27][16] (tap-major, the layout seg3d_conv3d_cin1_fwd reads).  gy and w 16-byte aligned. */
+int seg3d_conv3d_cin1_dgrad(int dtype, const void* gy, int ld, const float* w, float* dx,
+                            int N, int D, int H, int W, void* stream);
+
 /* k3 s1 p1 convolution with a narrow output (Cout = classes <= 7; vnet_outblock.py:13) on the tensor cores: the nine
  * in-plane taps are folded into the GEMM N dimension and summed in the epilogue (csrc/conv_tc_narrow.cu).
  * x: [N,D,H,W,Cin] f16/bf16, Cin in {16,32,64}, W % 8 == 0.  w (dtype): [3 kd][NP][Cin] with row (kh*3+kw)*Cout + co,
@@ -351,6 +358,15 @@ int seg3d_gather_pack(const seg3d_pack_entry* table, const int32_t* block_map, i
  *   p -= lr/(1-beta1^step) * m / (sqrt(v)/sqrt(1-beta2^step) + eps).       All pointers 16-byte aligned. */
 int seg3d_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n,
                     float lr, float beta1, float beta2, float eps, float weight_decay, int step, void* stream);
+/* the same update over n_ranges sub-ranges of the flat buffers, range k covering elements [offset, offset + n) with its own
+ * step count (its own bias corrections); elements outside every range are not touched.  `ranges` is HOST memory, read
+ * before the call returns; offsets are multiples of 4, ranges do not overlap. */
+typedef struct {
+  int64_t offset, n, step;
+} seg3d_adam_range;
+int seg3d_adam_step_ranges(float* param, const float* grad, float* exp_avg, float* exp_avg_sq,
+                           const seg3d_adam_range* ranges, int n_ranges, float lr, float beta1, float beta2,
+                           float eps, float weight_decay, void* stream);
 
 #ifdef __cplusplus
 }

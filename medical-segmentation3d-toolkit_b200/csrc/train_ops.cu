@@ -5,7 +5,9 @@
 //                       flipped / transposed data-gradient weights), and one more launch turns the kernel-layout weight
 //                       gradients back into parameter layout;
 //   seg3d_adam_step   : torch.optim.Adam's update (the reference's optimiser, lr / betas / eps / weight decay) over one flat
-//                       fp32 range holding every parameter of the network.
+//                       fp32 range holding every parameter of the network;
+//   seg3d_adam_step_ranges : the same update over a list of sub-ranges, each with its own step count (parameters without a
+//                       gradient are left out of the list and keep their values and moments, as torch.optim.Adam skips them).
 // Both are pure streaming kernels over ~58 MB; they replace ~250 tiny framework launches per step.
 #include "common.cuh"
 
@@ -53,11 +55,12 @@ gather_pack_kernel(const seg3d_pack_entry* __restrict__ table, const int32_t* __
 
 // torch/optim/adam.py::_single_tensor_adam (no amsgrad, no maximize):
 //   g += wd * p;  m.lerp_(g, 1 - b1);  v = b2 * v + (1 - b2) * g * g;  p -= step_size * m / (sqrt(v) / sqrt(bc2) + eps)
-__global__ void __launch_bounds__(256)
-adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long long n,
-                 float b1, float b2, float eps, float wd, float step_size, float bc2_sqrt) {
+// over elements [0, n) of one range, element i taken by thread `first` + k * `stride` of the grid
+__device__ __forceinline__ void adam_range(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
+                                           float* __restrict__ v, long long n, float b1, float b2, float eps, float wd,
+                                           float step_size, float bc2_sqrt, long long first, long long stride) {
   const long long n4 = n >> 2;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
+  for (long long i = first; i < n4; i += stride) {
     float4 pp = reinterpret_cast<float4*>(p)[i], gg = reinterpret_cast<const float4*>(g)[i];
     float4 mm = reinterpret_cast<float4*>(m)[i], vv = reinterpret_cast<float4*>(v)[i];
     float* pa = &pp.x; float* ga = &gg.x; float* ma = &mm.x; float* va = &vv.x;
@@ -70,13 +73,43 @@ adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __re
     }
     reinterpret_cast<float4*>(p)[i] = pp; reinterpret_cast<float4*>(m)[i] = mm; reinterpret_cast<float4*>(v)[i] = vv;
   }
-  for (long long i = (n4 << 2) + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+  for (long long i = (n4 << 2) + first; i < n; i += stride) {
     const float gr = wd != 0.f ? fmaf(wd, p[i], g[i]) : g[i];
     const float mi = m[i] + (1.f - b1) * (gr - m[i]);
     const float vi = fmaf(1.f - b2, gr * gr, b2 * v[i]);
     m[i] = mi; v[i] = vi;
     p[i] -= step_size * (mi / (sqrtf(vi) / bc2_sqrt + eps));
   }
+}
+
+__global__ void __launch_bounds__(256)
+adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long long n,
+                 float b1, float b2, float eps, float wd, float step_size, float bc2_sqrt) {
+  adam_range(p, g, m, v, n, b1, b2, eps, wd, step_size, bc2_sqrt, (long long)blockIdx.x * blockDim.x + threadIdx.x,
+             (long long)gridDim.x * blockDim.x);
+}
+
+// seg3d_adam_step_ranges: up to ADAM_RANGES_PER_LAUNCH ranges per launch, passed by value; blockIdx.y picks the range
+constexpr int ADAM_RANGES_PER_LAUNCH = 32;
+struct AdamRanges {
+  long long off[ADAM_RANGES_PER_LAUNCH], n[ADAM_RANGES_PER_LAUNCH];
+  float step_size[ADAM_RANGES_PER_LAUNCH], bc2_sqrt[ADAM_RANGES_PER_LAUNCH];
+};
+
+__global__ void __launch_bounds__(256)
+adam_ranges_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                   const AdamRanges r, float b1, float b2, float eps, float wd) {
+  const int k = blockIdx.y;
+  const long long o = r.off[k];
+  adam_range(p + o, g + o, m + o, v + o, r.n[k], b1, b2, eps, wd, r.step_size[k], r.bc2_sqrt[k],
+             (long long)blockIdx.x * blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x);
+}
+
+// the bias corrections of one step count, in double as torch computes them, rounded once to fp32
+void adam_corrections(float lr, float beta1, float beta2, long long step, float& step_size, float& bc2_sqrt) {
+  const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
+  step_size = (float)((double)lr / bc1);
+  bc2_sqrt = (float)sqrt(bc2);
 }
 
 }  // namespace
@@ -92,12 +125,40 @@ extern "C" int seg3d_adam_step(float* param, const float* grad, float* exp_avg, 
                                float lr, float beta1, float beta2, float eps, float weight_decay, int step, void* stream) {
   SEG3D_REQUIRE(param && grad && exp_avg && exp_avg_sq && n > 0 && step >= 1, "adam_step: bad arguments");
   SEG3D_REQUIRE(((uintptr_t)param | (uintptr_t)grad | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) % 16 == 0, "adam_step: pointers must be 16-byte aligned");
-  const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
-  const float step_size = (float)((double)lr / bc1), bc2_sqrt = (float)sqrt(bc2);
+  float step_size, bc2_sqrt;
+  adam_corrections(lr, beta1, beta2, step, step_size, bc2_sqrt);
   long long want = ((n >> 2) + 255) / 256;
   const int cap = 8 * seg3d_num_sms();
   const int gx = (int)(want < 1 ? 1 : (want > cap ? cap : want));
   adam_step_kernel<<<gx, 256, 0, (cudaStream_t)stream>>>(param, grad, exp_avg, exp_avg_sq, n, beta1, beta2, eps, weight_decay, step_size, bc2_sqrt);
   SEG3D_CHECK_LAUNCH("adam_step_kernel");
+  return SEG3D_OK;
+}
+
+extern "C" int seg3d_adam_step_ranges(float* param, const float* grad, float* exp_avg, float* exp_avg_sq,
+                                      const seg3d_adam_range* ranges, int n_ranges, float lr, float beta1, float beta2,
+                                      float eps, float weight_decay, void* stream) {
+  SEG3D_REQUIRE(param && grad && exp_avg && exp_avg_sq && ranges && n_ranges > 0, "adam_step_ranges: bad arguments");
+  SEG3D_REQUIRE(((uintptr_t)param | (uintptr_t)grad | (uintptr_t)exp_avg | (uintptr_t)exp_avg_sq) % 16 == 0,
+                "adam_step_ranges: pointers must be 16-byte aligned");
+  const int cap = 8 * seg3d_num_sms();
+  for (int r0 = 0; r0 < n_ranges; r0 += ADAM_RANGES_PER_LAUNCH) {
+    const int nr = n_ranges - r0 < ADAM_RANGES_PER_LAUNCH ? n_ranges - r0 : ADAM_RANGES_PER_LAUNCH;
+    AdamRanges t;
+    long long longest = 0;
+    for (int k = 0; k < nr; ++k) {
+      const seg3d_adam_range& e = ranges[r0 + k];
+      SEG3D_REQUIRE(e.offset >= 0 && e.offset % 4 == 0 && e.n > 0 && e.step >= 1,
+                    "adam_step_ranges: range %d needs offset >= 0 (a multiple of 4), n > 0 and step >= 1", r0 + k);
+      t.off[k] = e.offset; t.n[k] = e.n;
+      adam_corrections(lr, beta1, beta2, e.step, t.step_size[k], t.bc2_sqrt[k]);
+      longest = e.n > longest ? e.n : longest;
+    }
+    const long long want = ((longest >> 2) + 255) / 256;
+    const int per = (cap + nr - 1) / nr;
+    const int gx = (int)(want < 1 ? 1 : (want > per ? per : want));
+    adam_ranges_kernel<<<dim3(gx, nr), 256, 0, (cudaStream_t)stream>>>(param, grad, exp_avg, exp_avg_sq, t, beta1, beta2, eps, weight_decay);
+    SEG3D_CHECK_LAUNCH("adam_ranges_kernel");
+  }
   return SEG3D_OK;
 }

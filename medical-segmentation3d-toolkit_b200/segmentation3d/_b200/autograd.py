@@ -2,7 +2,9 @@
 `outputs = net(crops); loss.backward()`).
 
 Forward = the same kernel plan as inference, built in `train` mode so every pre-GroupNorm tensor and every
-activation is kept.  Backward walks the recorded conv->GN->ReLU units in reverse:
+activation is kept.  Backward walks the recorded conv->GN->ReLU units in reverse, issuing only what autograd asks for
+(_Backward.schedule: frozen weights get no weight gradient, a unit with nothing trainable at or upstream of it is skipped,
+the network input gets a gradient when it requires one):
 
     gn_bwd pass 0/1  (dz = g*[out>0], GroupNorm backward, dgamma/dbeta/dbias, residual gradient)
     conv wgrad       (seg3d_conv3d_wgrad, fp32 accumulation)
@@ -41,6 +43,7 @@ def unit_step(dt, B, gsrc, out, raw, C, stats, gamma, beta, sums, dgamma, dbeta,
                           `relu`; dy -> gy, dz -> dres (a unit with a residual), dgamma/dbeta/dbias
         conv wgrad        dw (kernel layout, fp32, accumulated) from the unit's input x (dims xd) and gy
         conv dgrad        dgrad = (dgrad convolution, gradient view, gy's dims), or None when no input gradient is needed
+    dw=None skips the weight gradient (a frozen convolution).
     `xpad` (whole network only): the input block's row-padded input, whose weight gradient has a kernel of its own."""
     st = lib.stream_ptr
     gv = list(gsrc) + [None] * (3 - len(gsrc))
@@ -55,7 +58,9 @@ def unit_step(dt, B, gsrc, out, raw, C, stats, gamma, beta, sums, dgamma, dbeta,
         for p in range(2):
             lib.call('seg3d_gn_bwd_noact', dt, p, *g, raw.p, raw.ld, C, stats, gamma, GN_EPS,
                      sums, dgamma, dbeta, gy.p, gy.ld, dres.p if dres else None, dres.ld if dres else 0, dbias, B, nvox, st())
-    if xpad is not None:
+    if dw is None:
+        pass
+    elif xpad is not None:
         lib.call('seg3d_conv3d_cin1_wgrad', dt, xpad.p, xd[2] + lib.CIN1_PAD, gy.p, gy.ld, dw, B, xd[0], xd[1], xd[2], st())
     else:
         lib.call('seg3d_conv3d_wgrad', mode, dt, x.p, x.ld, cin, gy.p, gy.ld, C, dw, B, xd[0], xd[1], xd[2], st())
@@ -114,17 +119,57 @@ class _Backward(object):
         tx = ws['tail']['x']
         self.gd_tail = _View(torch.empty((B, vox[0], tx.C), dtype=td, device=dev), 0, tx.C, tx.C)
         self.sums = torch.zeros((len(self.units) + 2, B, 2), dtype=torch.float64, device=dev)
+        self.schedules = {}
+        self.dconv_in, self.gd_in = None, None      # multi-channel input gradient, built when first asked for (_input_dgrad)
         self._make_dgrad_convs()
         self._make_tables()
 
     def _has_producer(self, x):
         return any(id(x.buf) == k[0] and x.off <= k[1] < x.off + x.C for k in self.produced)
 
+    def _inside(self, xv):
+        """keys of the producers inside consumer input window xv (the channel-span rule of add_contrib)"""
+        return [(bid, off) for (bid, off), pv in self.produced.items()
+                if bid == id(xv.buf) and xv.off <= off and off + pv.C <= xv.off + xv.C]
+
+    def schedule(self, need_input, need):
+        """What the walk issues for one gradient mask (need_input: the network input needs a gradient; need: the names of
+        the parameters that do), cached per mask.  A unit is needed when one of its parameters is trainable or a producer
+        inside its input (or residual) window is needed - for the input block, when the input needs a gradient.  A unit that
+        is not needed issues nothing; a needed one runs both GroupNorm backward passes, its weight gradient only when its
+        conv weight or bias is trainable, and its data gradient only when its input needs one.  The out-block tail follows
+        the same rule.  Returns {'units': [(run, wgrad, dgrad)], 'tail': (run, wgrad, dgrad), 'slots': (lo, hi)}, where
+        [lo, hi) is the range of the flat parameter-gradient buffer that holds the trainable parameters."""
+        key = (bool(need_input), frozenset(need))
+        sched = self.schedules.get(key)
+        if sched is not None:
+            return sched
+        needed, units = {}, []
+        for u in self.units:
+            conv_t = u['conv'] + '.weight' in need or u['conv'] + '.bias' in need
+            gn_t = u['gn'] + '.weight' in need or u['gn'] + '.bias' in need
+            if u['conv'] == 'in_block.conv':
+                dgrad = bool(need_input)
+            else:
+                dgrad = any(needed[k] for k in self._inside(u['x']))
+            res = u['res'] is not None and any(needed[k] for k in self._inside(u['res']))
+            run = conv_t or gn_t or dgrad or res
+            needed[(id(u['out'].buf), u['out'].off)] = run
+            units.append((run, run and conv_t, dgrad))
+        tail_t = any(k.startswith('out_block.') for k in need)
+        tail_dgrad = any(needed[k] for k in self._inside(self.ws['tail']['x']))
+        tail_w = 'out_block.conv1.weight' in need or 'out_block.conv1.bias' in need
+        tail_run = tail_t or tail_dgrad
+        ends = [(self.pg_off[k], self.pg_off[k] + self.pgrad[k].numel()) for k in need if k in self.pg_off]
+        slots = (min(a for a, _ in ends), max(b for _, b in ends)) if ends else (0, 0)
+        sched = self.schedules[key] = {'units': units, 'tail': (tail_run, tail_run and tail_w, tail_dgrad), 'slots': slots}
+        return sched
+
     def _make_dgrad_convs(self):
         plan = self.plan
         sd = self._weights()
         for name, c in list(plan.convs.items()):
-            if name == 'in_block.conv':
+            if name == 'in_block.conv':     # the network input's gradient: _input_grad
                 continue
             if c.mode == lib.CONV_K3:
                 pad = c.cout if c.cout != c.real_cout else 0
@@ -184,6 +229,8 @@ class _Backward(object):
         self.unpack_table = u
 
     def refresh(self):
+        if self.dconv_in is not None:
+            self.dconv_in.load(self._weights())
         if self.pack_table is not None and self.plan._bound_valid():
             self.pack_table.run()
             return
@@ -191,23 +238,42 @@ class _Backward(object):
         for c in self.dconv.values():
             c.load(sd)
 
-    # --------------------------------------------------------------------------------------------
-    def run(self, dprobs):
+    def _input_dgrad(self):
+        """(dgrad convolution, gradient view, gy dims) of a multi-channel network input's gradient, built on first use so that
+        a step that does not ask for it re-packs and allocates nothing for it"""
         plan, ws = self.plan, self.ws
+        if self.dconv_in is None:
+            self.dconv_in = _Conv(self._weights(), 'in_block.conv', lib.CONV_K3, plan.dt, plan.device, plan.tc_modes,
+                                  transform=_k3_dgrad_weight)
+            C = plan.in_channels
+            self.gd_in = _View(torch.empty((ws['B'], ws['vox'][0], C), dtype=plan.tdtype, device=plan.device), 0, C, C)
+        return self.dconv_in, self.gd_in, ws['dims'][0]
+
+    # --------------------------------------------------------------------------------------------
+    def run(self, dprobs, need_input=False, need=None):
+        """-> (parameter gradients by name, input gradient or None).  need: the parameter names that need a gradient
+        (None: every parameter); the gradients of the others are not computed and must not be used."""
+        plan, ws = self.plan, self.ws
+        if need is None:
+            need = self.pgrad.keys()
+        sched = self.schedule(need_input, need)
+        slot_lo, slot_hi = sched['slots']
         B, vox, dims, dt = ws['B'], ws['vox'], ws['dims'], plan.dt
         st = lib.stream_ptr
         self.pgrad_flat.zero_()
         self.sums.zero_()
         contrib = {}
         # data parallel: the slots are laid out in forward order and the walk below finishes them back to front, so the
-        # finished tail of the flat buffer is all-reduced (NCCL, its own stream) while the rest of the backward pass runs
+        # finished tail of the flat buffer is all-reduced (NCCL, its own stream) while the rest of the backward pass runs.
+        # Only the slots of trainable parameters, [slot_lo, slot_hi), are reduced.
         _, world = D.world()
         overlap = world > 1 and os.environ.get('SEG3D_OVERLAP_ALLREDUCE', '1') != '0'
-        works, sent_lo = [], self.pg_total
+        works, sent_lo = [], slot_hi
         bucket = int(os.environ.get('SEG3D_ALLREDUCE_BUCKET_MB', '12')) << 18          # floats
 
         def reduce_tail(lo, force=False):
             nonlocal sent_lo
+            lo = max(lo, slot_lo)
             if overlap and sent_lo > lo and (force or sent_lo - lo >= bucket):
                 works.append(torch.distributed.all_reduce(self.pgrad_flat[lo:sent_lo], op=torch.distributed.ReduceOp.SUM,
                                                           async_op=True))
@@ -230,7 +296,8 @@ class _Backward(object):
         sums2, sums1 = lib.ptr(self.sums[nu]), lib.ptr(self.sums[nu + 1])
         pg = self.pgrad
         dp = dprobs.contiguous().float()
-        for p in range(3):
+        tail_run, tail_w, tail_dgrad = sched['tail']
+        for p in range(3 if tail_run else 0):
             lib.call('seg3d_outblock_tail_bwd', dt, p, tail['raw'].p, tail['raw'].ld, nc, s1, lib.ptr(g1.gamma), lib.ptr(g1.beta),
                      lib.ptr(plan.w2), lib.ptr(plan.b2), s2, lib.ptr(g2.gamma), lib.ptr(g2.beta), GN_EPS, lib.ptr(dp),
                      sums2, sums1, lib.ptr(pg['out_block.gn2.weight']), lib.ptr(pg['out_block.gn2.bias']),
@@ -239,17 +306,23 @@ class _Backward(object):
                      self.gy_tail.p, self.gy_tail.ld, B, vox[0], st())
         x = tail['x']
         d0 = dims[0]
-        lib.call('seg3d_conv3d_wgrad', lib.CONV_K3, dt, x.p, x.ld, x.C, self.gy_tail.p, self.gy_tail.ld, self.conv1_co,
-                 lib.ptr(pg['out_block.conv1.weight']), B, d0[0], d0[1], d0[2], st())
-        dc = self.dconv['out_block.conv1']
-        lib.call('seg3d_conv3d_fwd', lib.CONV_K3, dt, dc.impl, self.gy_tail.p, self.gy_tail.ld, dc.cin, lib.ptr(dc.w), None,
-                 self.gd_tail.p, self.gd_tail.ld, dc.cout, B, d0[0], d0[1], d0[2], None, st())
-        add_contrib(x, self.gd_tail)
+        if tail_w:
+            lib.call('seg3d_conv3d_wgrad', lib.CONV_K3, dt, x.p, x.ld, x.C, self.gy_tail.p, self.gy_tail.ld, self.conv1_co,
+                     lib.ptr(pg['out_block.conv1.weight']), B, d0[0], d0[1], d0[2], st())
+        if tail_dgrad:
+            dc = self.dconv['out_block.conv1']
+            lib.call('seg3d_conv3d_fwd', lib.CONV_K3, dt, dc.impl, self.gy_tail.p, self.gy_tail.ld, dc.cin, lib.ptr(dc.w), None,
+                     self.gd_tail.p, self.gd_tail.ld, dc.cout, B, d0[0], d0[1], d0[2], None, st())
+            add_contrib(x, self.gd_tail)
         reduce_tail(self.pg_off['out_block.conv1.weight'])
 
         # ---- conv -> GN -> ReLU units in reverse ---------------------------------------------------
+        dx = None
         for ui in range(nu - 1, -1, -1):
             u = self.units[ui]
+            run, wgrad, need_dgrad = sched['units'][ui]
+            if not run:
+                continue
             c = plan.convs[u['conv']]
             gsrc = contrib.get((id(u['out'].buf), u['out'].off), [])
             assert 1 <= len(gsrc) <= 3, (u['conv'], len(gsrc))
@@ -258,25 +331,46 @@ class _Backward(object):
             gy = self.gy[u['conv']]
             dres = self.dres.get(u['conv'])
             dgrad = None
-            if u['conv'] in self.gd:           # the dgrad convolution's input is dy, living at the unit's output level
+            if need_dgrad and u['conv'] in self.gd:    # the dgrad convolution's input is dy, living at the unit's output level
                 dgrad = (self.dconv[u['conv']], self.gd[u['conv']], dims[u['lout']])
+            elif need_dgrad and u['conv'] == 'in_block.conv' and plan.in_channels > 1:
+                dgrad = self._input_dgrad()
             # input block on the row-padded input (Toeplitz operands)
             xpad = u['xpad'] if u.get('xpad') is not None and gy.ld == 16 else None
             unit_step(dt, B, gsrc, u['out'], u['raw'], c.cout, sf, lib.ptr(gnp.gamma), lib.ptr(gnp.beta), lib.ptr(self.sums[ui]),
                       lib.ptr(pg[u['gn'] + '.weight']), lib.ptr(pg[u['gn'] + '.bias']), gy, dres, lib.ptr(pg[u['conv'] + '.bias']),
-                      vox[u['lout']], c.mode, u['x'], c.cin, lib.ptr(pg[u['conv'] + '.weight']), dims[u['lin']], dgrad, xpad=xpad)
+                      vox[u['lout']], c.mode, u['x'], c.cin, lib.ptr(pg[u['conv'] + '.weight']) if wgrad else None,
+                      dims[u['lin']], dgrad, xpad=xpad)
             if dres is not None:
                 add_contrib(u['res'], dres)
-            if dgrad is not None:
+            if u['conv'] == 'in_block.conv' and need_dgrad:
+                dx = self._input_grad(gy, dgrad)
+            elif dgrad is not None:
                 add_contrib(u['x'], dgrad[1])
             reduce_tail(self.pg_off[u['conv'] + '.weight'])
-        reduce_tail(0, force=True)
+        reduce_tail(slot_lo, force=True)
         for w in works:
             w.wait()
         self.grads_reduced = bool(works)
         if works:
             self.pgrad_flat.mul_(1.0 / world)
-        return self._param_grads()
+        return self._param_grads(), dx
+
+    def _input_grad(self, gy, dgrad):
+        """NCDHW fp32 gradient of the network input from the input block's conv-output gradient gy: one
+        seg3d_conv3d_cin1_dgrad for a single-channel input, else the generic data-gradient convolution (already issued by
+        unit_step into dgrad's view) turned into NCDHW by seg3d_grad_to_ncdhw.  It is not part of the flat parameter buffer."""
+        plan, ws = self.plan, self.ws
+        B, (D, H, W) = ws['B'], ws['dims'][0]
+        dx = torch.empty((B, plan.in_channels, D, H, W), dtype=torch.float32, device=plan.device)
+        if plan.in_channels == 1:
+            lib.call('seg3d_conv3d_cin1_dgrad', plan.dt, gy.p, gy.ld, lib.ptr(plan.convs['in_block.conv'].w), lib.ptr(dx),
+                     B, D, H, W, lib.stream_ptr())
+        else:
+            gd = dgrad[1]
+            lib.call('seg3d_grad_to_ncdhw', plan.dt, 1, lib.ptr(gd.buf), gd.ld, gd.off, None, 0, 0, None, 0, 0, plan.in_channels,
+                     B, D * H * W, lib.ptr(dx), lib.stream_ptr())
+        return dx
 
     def _param_grads(self):
         """kernel-layout fp32 gradients -> the reference's parameter layouts: one seg3d_gather_pack launch into a flat buffer
@@ -336,13 +430,15 @@ class _NetFunction(torch.autograd.Function):
             bw = ws['bwd'] = _Backward(plan, ws)
         else:
             bw.refresh()
-        grads = bw.run(dprobs)
+        need = {n for n, f in zip(ctx.names, ctx.needs_input_grad[3:]) if f}
+        grads, dx = bw.run(dprobs, ctx.needs_input_grad[1], need)
         plan.grads_reduced_in_backward = bw.grads_reduced       # train_step then skips its own all-reduce
-        # the slots are reused next step: hand autograd its own copy (one copy, in the reference's parameter layout)
+        # the slots are reused next step: hand autograd its own copy (one copy, in the reference's parameter layout);
+        # frozen parameters get None
         if bw.unpack_table is not None:
-            return (None, None, None) + tuple(grads[n] for n in ctx.names)          # already views of a private flat copy
-        return (None, None, None) + tuple(g.clone() if g.is_contiguous() else g.contiguous()
-                                          for g in (grads[n] for n in ctx.names))
+            return (None, dx, None) + tuple(grads[n] if n in need else None for n in ctx.names)   # views of a private flat copy
+        return (None, dx, None) + tuple((g.clone() if g.is_contiguous() else g.contiguous()) if n in need else None
+                                        for n, g in ((n, grads[n]) for n in ctx.names))
 
 
 def train_forward(net, x):

@@ -30,6 +30,7 @@ _SIGNATURES = {
     'seg3d_conv3d_fwd': (_i, [_i, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     'seg3d_conv3d_cin1_fwd': (_i, [_i, _i, _vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _f, _vp]),
     'seg3d_conv3d_cin1_wgrad': (_i, [_i, _vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _vp]),
+    'seg3d_conv3d_cin1_dgrad': (_i, [_i, _vp, _i, _vp, _vp, _i, _i, _i, _i, _vp]),
     'seg3d_conv3d_k3_narrow_np': (_i, [_i]),
     'seg3d_conv3d_k3_narrow_fwd': (_i, [_i, _vp, _i, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp]),
     'seg3d_conv3d_k3_gnin_fwd': (_i, [_i, _vp, _i, _i, _i, _vp, _vp, _vp, _f, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
@@ -70,6 +71,7 @@ _SIGNATURES = {
                                      _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i64, _vp]),
     'seg3d_gather_pack': (_i, [_vp, _vp, _i, _vp]),
     'seg3d_adam_step': (_i, [_vp, _vp, _vp, _vp, _i64, _f, _f, _f, _f, _f, _i, _vp]),
+    'seg3d_adam_step_ranges': (_i, [_vp, _vp, _vp, _vp, _vp, _i, _f, _f, _f, _f, _f, _vp]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 
@@ -79,6 +81,11 @@ class PackEntry(ctypes.Structure):
     _fields_ = [('src', ctypes.c_void_p), ('dst', ctypes.c_void_p), ('src_base', ctypes.c_int64), ('dst_base', ctypes.c_int64),
                 ('src_stride', ctypes.c_int64 * 5), ('dst_stride', ctypes.c_int64 * 5),
                 ('size', ctypes.c_int32 * 5), ('limit', ctypes.c_int32 * 5), ('dtype', ctypes.c_int32), ('kind', ctypes.c_int32)]
+
+
+class AdamRange(ctypes.Structure):
+    """seg3d_adam_range of include/seg3d_b200.h"""
+    _fields_ = [('offset', ctypes.c_int64), ('n', ctypes.c_int64), ('step', ctypes.c_int64)]
 
 
 PACK_PLAIN, PACK_SPLIT_HI, PACK_SPLIT_LO = 0, 1, 2

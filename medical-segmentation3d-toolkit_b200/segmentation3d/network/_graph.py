@@ -164,7 +164,9 @@ class VShapedNet(nn.Module):
 
     def forward(self, input):
         _plan._require_cuda(input.device, 'segmentation3d (B200 build) has no CPU path: pass a CUDA tensor')
-        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+        # differentiable when grad mode is on and the input or any parameter requires grad (the standalone modules' rule):
+        # frozen parameters get no gradient and an input that requires grad gets one
+        if torch.is_grad_enabled() and (input.requires_grad or any(p.requires_grad for p in self.parameters())):
             from segmentation3d._b200.autograd import train_forward
             return train_forward(self, input)
         with torch.no_grad():
